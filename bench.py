@@ -423,7 +423,7 @@ def bench_allocate(impl: str, quick: bool = False) -> dict:
     import logging
     import resource
     import shutil
-    import tempfile
+    from gpushare_device_plugin_b200.testing import socket_dir
     soft, hard = resource.getrlimit(resource.RLIMIT_NOFILE)  # c = 1 024 needs > 2 048 descriptors in the in-process arms
     if soft < hard:
         resource.setrlimit(resource.RLIMIT_NOFILE, (hard, hard))
@@ -439,7 +439,7 @@ def bench_allocate(impl: str, quick: bool = False) -> dict:
            "sweep": []}
 
     def start(n_pods, mod, gsbd_extra=()):
-        tmp = tempfile.mkdtemp(prefix="gsb-alloc-")
+        tmp = socket_dir("gsb-alloc-")
         kube = subprocess.Popen(mock_argv + ["--node", node, "--pods", str(n_pods)] + (["--mod"] if mod else []),
                                 stdin=subprocess.PIPE, stdout=subprocess.PIPE, text=True, cwd=ROOT)
         url = f"http://127.0.0.1:{int(kube.stdout.readline())}"
@@ -593,10 +593,11 @@ def pctl(sorted_ns, q):
     return sorted_ns[min(len(sorted_ns) - 1, int(q * len(sorted_ns)))]
 
 
-def timed_cycles(cyc, steps: int, warmup: int, dist, local, sampler=None):
+def timed_cycles(cyc, steps: int, warmup: int, dist, local, sampler=None, capture=None):
     """W warm-up steps, then exactly `steps` steps bracketed by barrier + synchronize; per-step host times kept.
     `sampler` (clocks) runs from before the warm-up to after the last step; the clock samples kept are those taken
-    while the GPU was under this load."""
+    while the GPU was under this load. `capture(cyc)`, if given, runs once the timed region is closed and before any
+    further step, and its result is returned as "captured"."""
     if sampler is not None:
         sampler.start()
     for _ in range(warmup):
@@ -623,6 +624,7 @@ def timed_cycles(cyc, steps: int, warmup: int, dist, local, sampler=None):
     wall_ns = time.perf_counter_ns() - t0
     barrier_sync(dist, local)
     close_ns = time.perf_counter_ns() - t0 - wall_ns
+    captured = capture(cyc) if capture is not None else None
     if sampler is not None:
         # the timed region is over (wall_ns is taken): a few more steps of the same load so that even a 7 ms
         # region is covered by samples taken at this clock/power state
@@ -632,7 +634,33 @@ def timed_cycles(cyc, steps: int, warmup: int, dist, local, sampler=None):
             sampler.sample_now()
     per_step.sort()
     return {"wall_ns": wall_ns, "closing_barrier_ns": close_ns, "kernel_ns": kernel_ns, "inventory_ns": inv_ns, "launches": steps, "last": r,
-            "p50_ms": pctl(per_step, 0.5) / 1e6, "p99_ms": pctl(per_step, 0.99) / 1e6, "max_ms": per_step[-1] / 1e6}
+            "p50_ms": pctl(per_step, 0.5) / 1e6, "p99_ms": pctl(per_step, 0.99) / 1e6, "max_ms": per_step[-1] / 1e6,
+            "captured": captured}
+
+
+def cycle_outputs(cyc, idx: int, arena: int, window: int) -> dict:
+    """What the cycler's last gsb_cycle handed its caller, as arrays for --dump-outputs:
+      list_and_watch  the ListAndWatchResponse bytes (float32, one byte per element), the card's UUID in them replaced
+                      by GPU-00000000-0000-0000-0000-000000000000 so that runs on different cards compare
+      inventory       [total_mib, slices]
+      probe           [healthy, mismatch_words, mismatch_bits, checksum_xor, checksum_sum, bytes_walked, window_offset]
+      window_sample   (64, 16384) 32-bit lanes of the window the cycle's VERIFY_REFILL rewrote, read back from HBM at
+                      64 KiB chunks chosen by a fixed seed
+    The window rotates over the arena, so with the same arguments the arrays repeat where the arena has the same size."""
+    import numpy as np
+    from gpushare_device_plugin_b200 import device
+    r, p = cyc.res, cyc.res.probe
+    n_win = arena // window if window < arena else 1
+    offset = ((cyc.cycle_no - 1) % n_win) * window  # the window gsb_cycle walks for this cycle_no
+    chunk = 64 << 10
+    starts = np.sort(np.random.default_rng(0).choice(p.bytes_walked // chunk, 64, replace=False)) * chunk
+    sample = [np.frombuffer(device.arena_read(idx, offset + int(a), chunk), dtype=np.uint32) for a in starts]
+    lw = cyc.list_and_watch_bytes().replace(r.info.uuid, b"GPU-00000000-0000-0000-0000-000000000000")
+    return {"list_and_watch": np.frombuffer(lw, dtype=np.uint8).astype(np.float32),
+            "inventory": np.array([r.info.total_mib, r.slices], dtype=np.float64),
+            "probe": np.array([r.healthy, p.mismatch_words, p.mismatch_bits, p.checksum_xor, p.checksum_sum,
+                               p.bytes_walked, offset], dtype=np.float64),
+            "window_sample": np.stack(sample).astype(np.float64)}
 
 
 def node_cycle_leg(device, n: int, steps: int, warmup: int, window: int) -> dict:
@@ -724,7 +752,8 @@ def bench_ours(args) -> None:
     sampler = ClockSampler(idx)
     # ---- headline: steady-state rotating window ------------------------------------------------
     cyc = device.Cycler(idx, window_bytes=window, variant=variant)
-    head = timed_cycles(cyc, args.steps, args.warmup, dist, local, sampler)
+    capture = (lambda c: cycle_outputs(c, idx, arena, window)) if args.dump_outputs and rank == 0 else None
+    head = timed_cycles(cyc, args.steps, args.warmup, dist, local, sampler, capture)
     clocks = sampler.stop()
     last = head["last"]
     snapshot_age_ms = last.snapshot_age_ns / 1e6
@@ -864,6 +893,11 @@ def bench_ours(args) -> None:
             line["allocate"]["python_front_end"] = bench_allocate("ours_py", True)
         except Exception as e:  # noqa: BLE001
             line["allocate"] = {"error": str(e)}
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in head["captured"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line))
 
 
@@ -889,7 +923,11 @@ def main():
     ap.add_argument("--quick-allocate", action="store_true")
     ap.add_argument("--allocate-only", action="store_true", help="host-only: print just the Allocate() leg")
     ap.add_argument("--allocate-impl", default="", choices=["", "ours", "ours_py", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the headline cycle returned in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.allocate_only):
+        ap.error("--dump-outputs writes the outputs of our arm's headline cycle")
     if args.warmup < 3:
         args.warmup = 3
     if args.allocate_only:

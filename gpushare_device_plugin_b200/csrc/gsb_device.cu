@@ -214,6 +214,9 @@ struct Global {
   std::vector<uint8_t> join_bits;
 
   // health
+  // serialises gsb_health_start, gsb_health_stop and gsb_shutdown, so that one call's threads and event set are never
+  // torn down by another's, nor devices freed under probers still running; taken before api_mu, never after it
+  std::mutex life_mu;
   std::mutex hmu;
   std::condition_variable hcv;
   std::deque<gsb_event> events;
@@ -878,6 +881,34 @@ void push_event(const gsb_event &ev) {
   G.hcv.notify_all();
 }
 
+void wake_health_waiters() {  // whether or not the internal threads are running
+  {
+    std::lock_guard<std::mutex> lk(G.hmu);
+    G.stop_gen++;
+  }
+  G.hcv.notify_all();
+}
+
+int health_stop_locked() {  // the caller holds G.life_mu
+  std::vector<std::thread> ts;
+  {
+    std::lock_guard<std::mutex> lk(G.mu);
+    if (!G.health_running) return GSB_OK;
+    G.health_stop = true;
+    ts.swap(G.health_threads);
+    G.health_running = false;
+  }
+  for (auto &t : ts) t.join();
+  if (G.have_event_set) {
+    G.ml.eventSetFree(G.event_set);
+    G.have_event_set = false;
+  }
+  std::lock_guard<std::mutex> lk(G.hmu);
+  G.events.clear();
+  G.health_stop = false;
+  return GSB_OK;
+}
+
 }  // namespace
 
 // ====================================================================== C ABI
@@ -984,7 +1015,9 @@ int gsb_init(void) {
 }
 
 int gsb_shutdown(void) {
-  gsb_health_stop();
+  wake_health_waiters();
+  std::lock_guard<std::mutex> life_lk(G.life_mu);
+  health_stop_locked();
   std::unique_lock<std::shared_mutex> api_lk(G.api_mu);  // waits for in-flight calls of other threads
   std::lock_guard<std::mutex> lk(G.mu);
   if (!G.inited) return GSB_OK;
@@ -1454,6 +1487,7 @@ int gsb_health_wait(uint32_t timeout_ms, gsb_event *ev) {
 }
 
 int gsb_health_start(uint32_t probe_period_ms, uint64_t window_bytes) {
+  std::lock_guard<std::mutex> life_lk(G.life_mu);
   std::shared_lock<std::shared_mutex> api_lk(G.api_mu);
   if (!G.inited) return GSB_ERR_NOT_INITIALIZED;
   std::lock_guard<std::mutex> lk(G.mu);
@@ -1616,28 +1650,9 @@ int gsb_health_start(uint32_t probe_period_ms, uint64_t window_bytes) {
 }
 
 int gsb_health_stop(void) {
-  {  // wake every waiter, whether or not the internal threads are running
-    std::lock_guard<std::mutex> lk(G.hmu);
-    G.stop_gen++;
-  }
-  G.hcv.notify_all();
-  std::vector<std::thread> ts;
-  {
-    std::lock_guard<std::mutex> lk(G.mu);
-    if (!G.health_running) return GSB_OK;
-    G.health_stop = true;
-    ts.swap(G.health_threads);
-    G.health_running = false;
-  }
-  for (auto &t : ts) t.join();
-  if (G.have_event_set) {
-    G.ml.eventSetFree(G.event_set);
-    G.have_event_set = false;
-  }
-  std::lock_guard<std::mutex> lk(G.hmu);
-  G.events.clear();
-  G.health_stop = false;
-  return GSB_OK;
+  wake_health_waiters();
+  std::lock_guard<std::mutex> life_lk(G.life_mu);
+  return health_stop_locked();
 }
 
 }  // extern "C"

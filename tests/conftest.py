@@ -22,6 +22,21 @@ def pytest_configure(config):
             subprocess.run(["bash", os.path.join(ROOT, "build.sh")], check=True, cwd=ROOT)
 
 
+@pytest.fixture
+def tmp_path(tmp_path):
+    """pytest's tmp_path, or, where that is too deep for the unix sockets the tests create in it (a socket's path may
+    not exceed 107 bytes: a long TMPDIR or user name), a fresh short directory that is removed afterwards."""
+    if len(str(tmp_path)) <= 72:
+        yield tmp_path
+        return
+    import pathlib
+    import shutil
+    from gpushare_device_plugin_b200.testing import socket_dir
+    d = socket_dir("gsb-test-")
+    yield pathlib.Path(d)
+    shutil.rmtree(d, ignore_errors=True)
+
+
 @pytest.fixture(scope="session")
 def gsb():
     """Initialised C-ABI device layer. GPU tests only; fails loudly (no CPU fallback exists)."""

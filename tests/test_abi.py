@@ -134,13 +134,15 @@ def test_plain_c99_client_sees_the_reference_bytes(tmp_path):
 
 def test_event_queue_and_lifecycle_under_concurrency(tmp_path):
     """tests/native/health_stress.cc: inject / wait / stop from many threads and the lifecycle entry points racing
-    each other, with no driver on the box. Every injected event is delivered exactly once; nothing crashes.
+    each other, with no device the library can use (on a GPU box CUDA_VISIBLE_DEVICES hides them, so no prober adds
+    events of its own). Every injected event is delivered exactly once; nothing crashes.
     (tools/sanitize.sh runs the same program against a TSan-instrumented build of the library.)"""
     exe = tmp_path / "health_stress"
     subprocess.run(["g++", "-O1", "-std=c++17", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", str(exe),
                     os.path.join(ROOT, "tests", "native", "health_stress.cc"), "-L", os.path.dirname(_abi.LIB_PATH),
                     "-lgpushare_b200", "-Wl,-rpath," + os.path.dirname(_abi.LIB_PATH)], check=True)
-    out = subprocess.run([str(exe), "1"], capture_output=True, text=True, timeout=60)
+    out = subprocess.run([str(exe), "1"], capture_output=True, text=True, timeout=60,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert out.returncode == 0, out.stdout + out.stderr
     f = dict(zip(out.stdout.split()[::2], map(int, out.stdout.split()[1::2])))
     assert f["injected"] == f["received"] > 1000 and f["lifecycle"] > 10 and f["stopped"] > 10

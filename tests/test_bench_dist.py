@@ -7,6 +7,8 @@ import socket
 import subprocess
 import sys
 
+from tests.ref_answers import recorded
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 WORKER = r'''
@@ -39,11 +41,18 @@ def launch(code_or_args, extra_env=None):
     port = free_port()
     procs = []
     for rank in range(2):
+        # no GPU in view: dist_setup takes NCCL and one GPU per rank wherever CUDA is available
         env = dict(os.environ, RANK=str(rank), LOCAL_RANK=str(rank), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1",
-                   MASTER_PORT=str(port), **(extra_env or {}))
+                   MASTER_PORT=str(port), CUDA_VISIBLE_DEVICES="", **(extra_env or {}))
         procs.append(subprocess.Popen([sys.executable] + code_or_args, env=env, stdout=subprocess.PIPE,
                                       stderr=subprocess.PIPE, text=True, cwd=ROOT))
-    outs = [p.communicate(timeout=180) for p in procs]
+    try:
+        outs = [p.communicate(timeout=180) for p in procs]
+    finally:
+        for p in procs:
+            if p.poll() is None:
+                p.kill()
+                p.wait()
     return procs, outs
 
 
@@ -65,8 +74,15 @@ def test_reference_arm_runs_on_rank0_only():
     line = json.loads(outs[0][0].strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["n_gpus"] == 2 and line["details"]["devices_seen"] == 2
     assert line["details"]["fake_devices"] == 358 and line["setup"]["register_calls"] == 179 * 4 + 179 * 6
+    ref = json.loads(recorded("ref_inventory_fake.json", ["bench", "--iters", "3", "--warmup", "1", "--gpus", "2"],
+                              {"FAKE_NVML_GPUS": "8"}).stdout)
+    assert (line["details"]["fake_devices"], line["details"]["lw_bytes"], line["setup"]["register_calls"]) == \
+        (ref["n_devices"], ref["lw_len"], ref["register_calls_per_setup"])
     assert set(line["details"]["phases"]["cycle_us"]) >= {"inventory_p50", "health_poll_p50", "cycle_mean"}
-    assert line["metric"] == "inventory+health-probe cycles/sec" and line["cpu_baseline"]["kind"] == "reference"
+    # the arm runs oracle/_ref/ref_inventory where `make -C oracle` could build it from the reference's sources,
+    # else the oracle port
+    kind = "reference" if os.access(os.path.join(ROOT, "oracle", "_ref", "ref_inventory"), os.X_OK) else "port"
+    assert line["metric"] == "inventory+health-probe cycles/sec" and line["cpu_baseline"]["kind"] == kind
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["value"] > 0
     assert outs[1][0].strip() == ""
     sys.path.insert(0, ROOT)

@@ -1,8 +1,10 @@
 """Pins the oracle itself (CPU): the numpy and C restatements of the probe spec against the committed
-golden vectors and against each other; the C restatement of the reference's NVML path (linked with
-the reference's own nvml_dl.c) against a fake libnvidia-ml with 8 synthetic B200s and against the
-pure-Python restatement of getDevices + gogo marshal."""
+golden vectors and against each other; the answers of the C restatement of the reference's NVML path
+(linked with the reference's own nvml_dl.c) against a fake libnvidia-ml with 8 synthetic B200s, as
+recorded in tests/golden/ref_inventory_fake.json, against the pure-Python restatement of getDevices +
+gogo marshal."""
 import ctypes as C
+import hashlib
 import json
 import os
 import subprocess
@@ -10,13 +12,13 @@ import subprocess
 import numpy as np
 import pytest
 
+from gpushare_device_plugin_b200 import _abi
 from oracle import probe_oracle as po
 from oracle import wire_oracle as wo
+from tests.ref_answers import recorded
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = json.load(open(os.path.join(ROOT, "tests", "golden", "probe_pattern.json")))
-REF_BIN = os.path.join(ROOT, "oracle", "_ref", "ref_inventory")
-FAKE = os.path.join(ROOT, "oracle", "_fake")
 
 
 def test_mix32_is_murmur3_finaliser():
@@ -70,30 +72,26 @@ def test_seeds_never_collide_and_addresses_are_unique():
 
 
 def run_ref(args, env_extra):
-    env = dict(os.environ, LD_LIBRARY_PATH=FAKE, **env_extra)
-    out = subprocess.run([REF_BIN] + args, env=env, capture_output=True, text=True)
-    return out
+    return recorded("ref_inventory_fake.json", args, env_extra)
 
 
-@pytest.mark.skipif(not os.access(REF_BIN, os.X_OK), reason="oracle/_ref not built (no /root/reference here)")
 class TestReferenceRestatement:
     def test_without_nvml_it_reports_the_reference_error(self):
-        if os.path.exists("/usr/lib/x86_64-linux-gnu/libnvidia-ml.so.1"):
-            pytest.skip("real NVML present")
-        out = subprocess.run([REF_BIN, "inventory"], capture_output=True, text=True)
+        out = run_ref(["inventory"], None)
         assert out.returncode == 12 and "could not load NVML library" in out.stderr  # bindings.go:60-66
+        assert _abi.lib.gsb_strerror(_abi.GSB_ERR_LIBRARY_NOT_FOUND).decode() in out.stderr  # the product says the same
 
     @pytest.mark.parametrize("n", [1, 2, 8])
-    def test_inventory_matches_python_restatement(self, n, tmp_path):
-        lw = tmp_path / "lw.bin"
-        out = run_ref(["inventory", "--lw-out", str(lw)], {"FAKE_NVML_GPUS": str(n)})
+    def test_inventory_matches_python_restatement(self, n):
+        out = run_ref(["inventory", "--lw-out"], {"FAKE_NVML_GPUS": str(n)})
         assert out.returncode == 0, out.stderr
         j = json.loads(out.stdout)
         assert (j["n_gpus"], j["gpu_memory"], j["n_devices"]) == (n, 179, 179 * n)
         devs, names, mem = wo.getDevices([{"uuid": d["uuid"], "path": d["path"], "memory_mib": d["memory_mib"]}
                                           for d in j["devices"]])
-        assert mem == 179 and lw.read_bytes() == wo.marshal_ListAndWatchResponse(devs)
-        assert len(lw.read_bytes()) == {1: 10451, 2: 20902, 8: 83608}[n]  # SURVEY.md §8(a) a7
+        lw = wo.marshal_ListAndWatchResponse(devs)
+        assert mem == 179 and hashlib.sha256(lw).hexdigest() == out.lw_sha256
+        assert len(lw) == j["lw_len"] == {1: 10451, 2: 20902, 8: 83608}[n]  # SURVEY.md §8(a) a7
         assert names == {d["uuid"]: d["minor"] for d in j["devices"]}
         assert all(d["memory_mib"] == 183359 and d["total_bytes"] == 192265846784 for d in j["devices"])
 
